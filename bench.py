@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   (also writes the last timed step's results: dump_outputs)
 
 Workload (config.workload): BASELINE.json configs[3] -- weighted rendezvous placement of 10 M objects x 1024 nodes
 (weights u32 in [1,16], seed 7; keys = splitmix stream), id-range sharded one shard per GPU, with the bounded-load
@@ -211,6 +212,30 @@ def pinned_array(p, nbytes, dtype):
     return arr, ptr
 
 
+DUMP_MAX_BYTES = 64 << 20   # all ranks' files together
+DUMP_SEED = 20240917
+
+
+def dump_outputs(out_dir, s, passes, rank, world):
+    """What a caller of the timed step receives, as .npy files a second build's run can be compared with file for file:
+    node_index (the node chosen for every object of the rank's shard, float32; 4294967296 = no node), load_counters (the global
+    per-node loads the capacity check saw, float64) and passes (float64).  A shard whose node_index would not fit this rank's
+    share of DUMP_MAX_BYTES is written as a seeded sample of it, the sampled object positions in node_index_position (float64).
+    With world > 1 every name ends in _rank<r>."""
+    os.makedirs(out_dir, exist_ok=True)
+    sfx = "_rank%d" % rank if world > 1 else ""
+    idx = s.read()
+    counters = s.counters()
+    budget = DUMP_MAX_BYTES // world - counters.size * 8 - 1024
+    out = {"node_index": idx, "load_counters": counters.astype(np.float64), "passes": np.array([passes], dtype=np.float64)}
+    if idx.size * 4 > budget:
+        pos = np.unique(np.random.default_rng(DUMP_SEED).integers(0, idx.size, budget // 12))
+        out["node_index"], out["node_index_position"] = idx[pos], pos.astype(np.float64)
+    out["node_index"] = out["node_index"].astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + sfx + ".npy"), a)
+
+
 def run_reference(args, rank, world):
     """The reference's own CPU path for this metric: per-id Service::get_or_create_placement over LocalObjectPlacement
     (service.rs:193-254, local.rs:12-68), all host threads, bounded sample per step."""
@@ -282,7 +307,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the C2/C3/C4-strong/C5 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -368,13 +396,14 @@ def main():
     DEPTH = max(1, min(N_SETS - 1, int(os.environ.get("RIO_BENCH_DEPTH", "3"))))
 
     def run_steps(k0, k):
-        passes = 1
+        """Steps k0 .. k0+k-1; returns the passes each one took, in step order."""
+        passes = []
         for i in range(k0, k0 + k):
             sets[i % N_SETS].assign_bounded_begin(n_global, 5, 4, 4)
             if i - k0 >= DEPTH:
-                passes = max(passes, sets[(i - DEPTH) % N_SETS].assign_bounded_end())
+                passes.append(sets[(i - DEPTH) % N_SETS].assign_bounded_end())
         for i in range(max(k0, k0 + k - DEPTH), k0 + k):
-            passes = max(passes, sets[i % N_SETS].assign_bounded_end())
+            passes.append(sets[i % N_SETS].assign_bounded_end())
         return passes
 
     # ONE sampler for the whole job (rank 0 watches every GPU of the run): a poller per rank contends for the driver
@@ -382,7 +411,7 @@ def main():
     clocks = ClockSampler(range(world)) if rank == 0 else None
     if clocks:
         clocks.start()
-    passes = run_steps(0, args.warmup)
+    passes = max([1] + run_steps(0, args.warmup))
     barrier_sync()
     if clocks:
         time.sleep(0.25)   # make sure the sampler is producing before the timed region starts
@@ -390,9 +419,12 @@ def main():
     barrier_sync()
     l0 = p.launch_count()
     p.event_record(0)
-    passes = max(passes, run_steps(args.warmup, args.steps))
+    timed_passes = run_steps(args.warmup, args.steps)
     p.event_record(1)
     barrier_sync()
+    passes = max([passes] + timed_passes)
+    if args.dump_outputs:   # before anything below reuses the resident sets
+        dump_outputs(args.dump_outputs, sets[(args.warmup + args.steps - 1) % N_SETS], timed_passes[-1], rank, world)
     my_ms = p.event_elapsed_ms(0, 1)
     ms_total = max_over_ranks(my_ms)
     per_rank_ms = None

@@ -72,17 +72,19 @@ def run(R, O, device=0, n=1000, M=4):
     p.lookup_many(big)
     out["gpu_batched_lookup_ns_per_id_1M_batch"] = 1e9 * (time.perf_counter() - t0) / len(big)
     assert (got == np.arange(n) % M).all()
-    # the same calls from real threads through the C ABI (the Python threads above serialise on the interpreter lock)
+    # the same calls from real threads through the C ABI (the Python threads above serialise on the interpreter lock); the
+    # harness is compiled into a temporary directory so that a benchmark run leaves the source tree as it found it (it may be read-only)
     try:
         import subprocess
+        import tempfile
 
-        exe = os.path.join(ROOT, "tools", "bench_c1")
         src = os.path.join(ROOT, "tools", "bench_c1.cpp")
         so_dir = os.path.join(ROOT, "rio_rs_b200")
-        if not os.path.exists(exe) or os.path.getmtime(exe) < os.path.getmtime(src):
+        with tempfile.TemporaryDirectory() as tmp:
+            exe = os.path.join(tmp, "bench_c1")
             subprocess.check_call(["g++", "-O2", "-std=c++17", "-pthread", src, "-I" + os.path.join(ROOT, "include"), "-L" + so_dir, "-lrio_cuda",
                                    "-Wl,-rpath," + so_dir, "-o", exe])
-        out["c_abi_threads"] = json.loads(subprocess.check_output([exe], timeout=300).decode().strip().splitlines()[-1])
+            out["c_abi_threads"] = json.loads(subprocess.check_output([exe], timeout=300).decode().strip().splitlines()[-1])
     except Exception as e:  # noqa: BLE001
         out["c_abi_threads"] = {"error": repr(e)}
     out["note"] = ("a per-id call is one GPU round trip (H2D 8 B, launch, D2H, sync): latency-bound; the per-request call sites are meant to go "
