@@ -69,6 +69,10 @@ def lib():
         L.orc_assign_bounded.argtypes = [u64p, C.c_size_t, u64p, u32p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, u32p, u32p, C.c_int]
         L.orc_assign_affinity.restype = None
         L.orc_assign_affinity.argtypes = [f32p, f32p, u32p, C.c_size_t, C.c_uint32, C.c_uint32, u32p, f64p, f64p, C.c_int]
+        L.orc_assign_affinity_f32.restype = None
+        L.orc_assign_affinity_f32.argtypes = [f32p, f32p, u32p, C.c_size_t, C.c_uint32, C.c_uint32, u32p, C.c_int]
+        L.orc_affinity_pair_cost_f32.restype = None
+        L.orc_affinity_pair_cost_f32.argtypes = [f32p, f32p, u32p, u32p, C.c_size_t, C.c_uint32, f32p, C.c_int]
         L.orc_assign_hrw2.restype = None
         L.orc_assign_hrw2.argtypes = [u64p, C.c_size_t, u64p, u32p, u32p, C.c_uint32, C.c_uint32, u32p, C.c_int]
         L.orc_assign_bounded_hrw2.restype = C.c_uint32
@@ -186,6 +190,32 @@ def assign_affinity(fobj, fnode, weights, threads=1):
     lib().orc_assign_affinity(_p(fobj, C.c_float), _p(fnode, C.c_float), _p(weights, C.c_uint32), n, M, K, _p(idx, C.c_uint32),
                               _p(cost, C.c_double), _p(gap, C.c_double), threads)
     return idx, cost, gap
+
+
+def assign_affinity_f32(fobj, fnode, weights, threads=1):
+    """Implementation restatement, not spec: the CUDA-core kernels' fp32 arithmetic (fmaf over k ascending, strict < in node
+    order).  Their indices must equal this exactly."""
+    fobj = np.ascontiguousarray(fobj, dtype=np.float32)
+    fnode = np.ascontiguousarray(fnode, dtype=np.float32)
+    weights = np.ascontiguousarray(weights, dtype=np.uint32)
+    n, K = fobj.shape
+    idx = np.empty(n, dtype=np.uint32)
+    lib().orc_assign_affinity_f32(_p(fobj, C.c_float), _p(fnode, C.c_float), _p(weights, C.c_uint32), n, fnode.shape[0], K, _p(idx, C.c_uint32),
+                                  threads)
+    return idx
+
+
+def affinity_pair_cost_f32(fobj, fnode, obj, node, threads=1):
+    """fp32 fmaf cost -sum_k fobj[obj[q],k] * fnode[node[q],k] for each pair q, with the arithmetic of assign_affinity_f32."""
+    fobj = np.ascontiguousarray(fobj, dtype=np.float32)
+    fnode = np.ascontiguousarray(fnode, dtype=np.float32)
+    obj = np.ascontiguousarray(obj, dtype=np.uint32)
+    node = np.ascontiguousarray(node, dtype=np.uint32)
+    assert obj.shape == node.shape and (obj < fobj.shape[0]).all() and (node < fnode.shape[0]).all()
+    out = np.empty(obj.shape, dtype=np.float32)
+    lib().orc_affinity_pair_cost_f32(_p(fobj, C.c_float), _p(fnode, C.c_float), _p(obj, C.c_uint32), _p(node, C.c_uint32), obj.size, fobj.shape[1],
+                                     _p(out, C.c_float), threads)
+    return out
 
 
 def counts(idx, M):

@@ -28,6 +28,7 @@
 #include <stddef.h>
 #include <stdlib.h>
 #include <string.h>
+#include <math.h>
 
 #define ORC_NONE 0xFFFFFFFFu
 
@@ -267,6 +268,48 @@ void orc_assign_affinity(const float *fobj, const float *fnode, const uint32_t *
                          uint32_t K, uint32_t *out_idx, double *out_cost, double *out_gap, int threads) {
     aff_ctx a = { fobj, fnode, weight, M, K, out_idx, out_cost, out_gap };
     par_for(n, threads, aff_range, &a);
+}
+
+/* ---- 3.6 in fp32 with the CUDA-core arithmetic: an IMPLEMENTATION RESTATEMENT, not spec ------------------------------
+ * The spec (above) is the fp64 argmin.  This restates what the CUDA-core kernels (k_assign_affinity, K = 16, and
+ * k_assign_affinity_generic) and the tensor-core path's fp32 re-scoring of its 8 candidates are specified to compute:
+ * acc = fmaf(Fobj[i,k], Fnode[j,k], acc) for k = 0..K-1 starting from +0.f, cost = -acc, strict < over the live nodes in
+ * index order (ties -> lowest j), ORC_NONE when no node is live.  libm fmaf is correctly rounded, so the chain is bit for
+ * bit the device's FFMA chain; an emulation in fp64 would round twice. */
+static float aff_cost_f32(const float *fo, const float *fn, uint32_t K) {
+    float acc = 0.f;
+    for (uint32_t k = 0; k < K; k++) acc = fmaf(fo[k], fn[k], acc);
+    return -acc;
+}
+static void aff_f32_range(void *p, size_t lo, size_t hi) {
+    aff_ctx *a = (aff_ctx *)p;
+    for (size_t i = lo; i < hi; i++) {
+        const float *fo = a->fobj + i * a->K;
+        float best = 0.f; uint32_t bj = ORC_NONE;
+        for (uint32_t j = 0; j < a->M; j++) {
+            if (!a->weight[j]) continue;
+            const float c = aff_cost_f32(fo, a->fnode + (size_t)j * a->K, a->K);
+            if (bj == ORC_NONE || c < best) { best = c; bj = j; }
+        }
+        a->out_idx[i] = bj;
+    }
+}
+void orc_assign_affinity_f32(const float *fobj, const float *fnode, const uint32_t *weight, size_t n, uint32_t M, uint32_t K,
+                             uint32_t *out_idx, int threads) {
+    aff_ctx a = { fobj, fnode, weight, M, K, out_idx, NULL, NULL };
+    par_for(n, threads, aff_f32_range, &a);
+}
+
+/* the same fp32 cost for given (object, node) pairs */
+typedef struct { const float *fobj, *fnode; const uint32_t *obj, *node; uint32_t K; float *out; } pair_ctx;
+static void pair_range(void *p, size_t lo, size_t hi) {
+    pair_ctx *c = (pair_ctx *)p;
+    for (size_t q = lo; q < hi; q++) c->out[q] = aff_cost_f32(c->fobj + (size_t)c->obj[q] * c->K, c->fnode + (size_t)c->node[q] * c->K, c->K);
+}
+void orc_affinity_pair_cost_f32(const float *fobj, const float *fnode, const uint32_t *obj, const uint32_t *node, size_t n_pairs, uint32_t K,
+                                float *out_cost, int threads) {
+    pair_ctx c = { fobj, fnode, obj, node, K, out_cost };
+    par_for(n_pairs, threads, pair_range, &c);
 }
 
 /* ---- synthetic inputs (SURVEY section 8d) --------------------------------------------------------- */

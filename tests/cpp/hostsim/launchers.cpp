@@ -10,6 +10,7 @@
 #include <sched.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <vector>
 
@@ -156,7 +157,7 @@ void launch_assign_affinity(const Launch &L, const float *fobj, uint64_t n, cons
         for (uint32_t j = 0; j < n_total; j++) {
             if (!live[j]) continue;
             float acc = 0.f;
-            for (uint32_t k = 0; k < K; k++) acc += fobj[i * K + k] * fnode[(size_t)j * K + k];
+            for (uint32_t k = 0; k < K; k++) acc = std::fmaf(fobj[i * K + k], fnode[(size_t)j * K + k], acc);   // the kernels' FFMA chain
             const float cost = -acc;
             if (bj == kNone || cost < best) { best = cost; bj = j; }   // ties -> lowest j
         }

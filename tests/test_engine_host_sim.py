@@ -60,12 +60,14 @@ def test_the_doubles_cover_every_launcher_and_nothing_in_the_product_knows_them(
 
 
 def test_gpu_test_bodies_pass_on_the_engine_host_logic(hostsim_so):
-    """tests/test_gpu_parity.py, test_gpu_hrw2.py and test_gpu_integration.py, unchanged, against the host-sim library: every
-    scenario but the 10 M x 1024 flat grid (10^10 pair hashes: minutes on a CPU) -- including all 10 M objects under HRW2."""
+    """tests/test_gpu_parity.py, test_gpu_hrw2.py, test_gpu_integration.py and test_gpu_affinity.py, unchanged, against the host-sim
+    library: every scenario but the 10 M x 1024 flat grid (10^10 pair hashes: minutes on a CPU) -- including all 10 M objects under
+    HRW2.  The affinity double has no tensor cores, so there every affinity case takes the CUDA-core branch and must equal the fp32
+    fmaf restatement of the oracle exactly; compaction, the capacity fallback, chunking and the counters are the engine's own."""
     env = dict(os.environ)
     env["RIO_HOSTSIM_LIBRARY"] = hostsim_so
     env["PYTHONPATH"] = os.path.join(ROOT, "tests") + os.pathsep + env.get("PYTHONPATH", "")
-    mods = [os.path.join(ROOT, "tests", m) for m in ("test_gpu_parity.py", "test_gpu_hrw2.py", "test_gpu_integration.py")]
+    mods = [os.path.join(ROOT, "tests", m) for m in ("test_gpu_parity.py", "test_gpu_hrw2.py", "test_gpu_integration.py", "test_gpu_affinity.py")]
     cmd = [sys.executable, "-m", "pytest"] + mods + ["-m", "gpu", "-p", "hostsim_plugin", "-q", "-x", "-p", "no:cacheprovider", "-k", "not test_full_size_10m_x_1024_properties"]
     try:
         import pytest_timeout  # noqa: F401  (a test blocked inside a C call is only stopped by the thread method)

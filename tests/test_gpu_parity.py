@@ -1,5 +1,6 @@
 """GPU parity tests (run under gpurun): every call goes through the C ABI of librio_cuda.so and is compared with the
-CPU oracle on the same seeded inputs.  Integer / index work is bit-exact; the float-cost path is within 1e-5 relative.
+CPU oracle on the same seeded inputs.  Integer / index work is bit-exact; the float-cost path's contract (DESIGN.md 3.6) is
+checked in tests/test_gpu_affinity.py, the affinity tests here are the older 1e-5-relative ones on well-conditioned inputs.
 
 Directory tests restate the reference's own tests against the GPU provider, exactly as a `mod gpu { ... }` block in
 rio-rs/tests/object_placement_backend.rs would.
@@ -262,7 +263,8 @@ def test_golden_vectors_on_gpu(gp):
 @pytest.mark.parametrize("K,M,n", [(16, 1024, 60000), (16, 37, 5001), (16, 64, 999), (16, 65, 7000), (16, 300, 20000), (16, 2000, 4000), (8, 64, 3000), (5, 9, 1000)])
 def test_affinity_cost_argmin(gp, oracle, K, M, n, variant):
     """cost = -dot, argmin (DESIGN.md 3.6).  K == 16 runs on the tensor cores (tcgen05, bf16x3 split) unless
-    RIO_AFFINITY_VARIANT=ffma or the node set does not fit shared memory (M = 2000); other K use CUDA cores."""
+    RIO_AFFINITY_VARIANT=ffma or more than 2048 nodes are live (M = 2000 still fits: 1998 live nodes pad to 2048); other K
+    use CUDA cores.  tests/test_gpu_affinity.py holds the exact and error-bounded checks of every dispatch branch."""
     rng = np.random.default_rng(11)
     fo = rng.uniform(-1, 1, (n, K)).astype(np.float32)
     fn = np.random.default_rng(13).uniform(-1, 1, (M, K)).astype(np.float32)
